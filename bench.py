@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            our arm (CUDA engine through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   also writes what the last timed step returned as DIR/*.npy
 
 Metric (BASELINE.json): "rollback frames/sec at 1M entities x 8-frame window".
 One step = one SyncTest tick of the stress-test world at steady state: the request vector
@@ -283,7 +284,11 @@ def run_ours(args):
     K, W = args.steps, max(3, args.warmup)
     eng = Engine(max_entities=n, max_depth=maxp, fps=60, device=local_rank,
                  flags=capi.BGR_CFG_SHARDED if sharded else 0, order_base=first_row)
-    build_world(eng, n, d, SEED + rank)
+    # started long before the timed region: nvidia-smi's start-up and first polls slow a 2 ms region by ~1 %
+    sampler = ClockSampler(local_rank)
+    if rank == 0:
+        sampler.start()
+    cols = build_world(eng, n, d, SEED + rank)
     stream = torch.cuda.ExternalStream(eng.stream(), device=dev)   # the stream the kernels are launched on
     slot_bytes = eng.slot_bytes()
     if sharded:
@@ -299,10 +304,7 @@ def run_ours(args):
     BT = min(BT, capi.BGR_MAX_REQUESTS // (2 * d + 2)) if d > 0 else 0                          # ... that fit one call
     K3 = (min(K, 400) // BT) * BT if BT > 1 else 0
     KT = 64                            # ticks of each traced leg (pipelined / synchronous)
-    # A short K (the driver's 20) makes one timed region ~2 ms: time EXACTLY K steps several times and report the median
-    # region, so that one clock / scheduling hiccup cannot set the number.  Every region is bracketed as the contract says.
-    R = max(1, min(5, 400 // max(1, K)))
-    ticks = pregenerate_ticks(fill + W + 2 * R * K + K + K2 + K3 + 2 * KT, d, maxp)
+    ticks = pregenerate_ticks(fill + W + 3 * K + K2 + K3 + 2 * KT, d, maxp)
     pos = [0]
 
     def take(k):
@@ -314,16 +316,20 @@ def run_ours(args):
     depth = 4 if sharded else 2     # un-collected submits kept queued on the GPU (hides the host loop / rank jitter)
 
     def run_pipelined(tick_list):
-        inflight = 0
+        """Returns the checksums bgr_collect handed back for the last tick."""
+        inflight, last = 0, []
         for arr, nreq, _, info, _ in tick_list:
             eng.submit_prepared(info, arr, nreq)
             inflight += 1
             if inflight > depth:
-                history.extend(eng.collect())
+                last = eng.collect()
+                history.extend(last)
                 inflight -= 1
         while inflight:
-            history.extend(eng.collect())
+            last = eng.collect()
+            history.extend(last)
             inflight -= 1
+        return last
 
     def barrier():
         torch.cuda.synchronize()
@@ -343,37 +349,28 @@ def run_ours(args):
 
     run_pipelined(take(fill + W))           # ring fill + warm-up (>= 3 steady-state ticks)
     barrier()
-    # ---------------- value: device-timed, K ticks back to back (median of R such regions) ----------------
-    sampler = ClockSampler(local_rank)
-    if rank == 0:
-        sampler.start()
-    regions = []
-    for _ in range(R):
-        tk = take(K)
-        l0 = eng.launch_count()
-        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        barrier()
-        ev0.record(stream)
-        run_pipelined(tk)
-        ev1.record(stream)
-        barrier()
-        regions.append((max_over_ranks(ev0.elapsed_time(ev1)), tk, eng.launch_count() - l0))
-    regions.sort(key=lambda r: r[0] / sum(t[2] for t in r[1]))
-    ms, timed, launches = regions[len(regions) // 2]
-    ms_all = [r[0] for r in regions]
+    # ---------------- value: device-timed, K ticks back to back ----------------
+    sampler.rows.clear()              # clocks of the timed legs only
+    timed = take(K)
+    l0 = eng.launch_count()
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    barrier()
+    ev0.record(stream)
+    last_checksums = run_pipelined(timed)
+    ev1.record(stream)
+    barrier()
+    ms = max_over_ranks(ev0.elapsed_time(ev1))
+    launches = eng.launch_count() - l0
     adv_total = sum(t[2] for t in timed)
     adv_per_tick = adv_total / K
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, cols, last_checksums)
     # ---------------- e2e: ONE synchronous bgr_handle_requests per tick, host arrays in / host checksums out ----------------
-    e2e_regions = []
-    for _ in range(R):
-        tk = take(K)
-        b = CallerBatch(tk)
-        barrier()
-        e2e_regions.append((max_over_ranks(b.run(caller, eng)), tk, b))
-        history.extend(b.checksums())
-    e2e_regions.sort(key=lambda r: r[0] / sum(t[2] for t in r[1]))
-    e2e_s, e2e_ticks, batch = e2e_regions[len(e2e_regions) // 2]
-    e2e_all = [r[0] for r in e2e_regions]
+    e2e_ticks = take(K)
+    batch = CallerBatch(e2e_ticks)
+    barrier()
+    e2e_s = max_over_ranks(batch.run(caller, eng))
+    history.extend(batch.checksums())
     clocks = sampler.stop() if rank == 0 else None
     e2e_p50_us = float(np.median(batch.per_tick) * 1e6)
     h2d = sum(C.sizeof(capi.bgr_request) * t[1] + C.sizeof(capi.bgr_session_info) for t in e2e_ticks) / K
@@ -569,9 +566,6 @@ def run_ours(args):
                        "max_prediction": maxp,
                        "columns": "Transform40+Velocity12+Ttl8+alive1 = 61 B/entity/slot", "checksum": "every saved frame",
                        "advances_per_step": adv_per_tick,
-                       "timed_regions": {"count": R, "reported": "median region", "value_ms": ms_all, "e2e_s": e2e_all,
-                                         "why": "each region times exactly K steps between barrier + synchronize; a short K is "
-                                                "repeated so that one hiccup cannot set the number"},
                        "l2": "inputs larger than L2: each tick reads 1 slot and writes 9 images of "
                        f"{slot_bytes/1e6:.0f} MB (ring {maxp} slots)", "path": "fused" if fused else "stepwise",
                        "value_is": "device-timed PIPELINED submits (bgr_submit_requests / bgr_collect, consecutive launches overlap); "
@@ -637,6 +631,31 @@ def run_ours(args):
         dist.destroy_process_group()
     if not consistent:
         sys.exit(3)
+
+
+DUMP_SAMPLE_ROWS = 1 << 18   # 72 B per sampled row across the dumped arrays: 19 MB at most
+
+
+def dump_outputs(out_dir, eng, cols, checksums):
+    """What the timed path handed back on its last step, as float arrays two builds can be compared with: the
+    (frame, checksum) pairs bgr_collect returned, and the live particle columns of a fixed, seeded sample of rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rows_total = eng.row_count()
+    rows = np.sort(np.random.default_rng(SEED).choice(rows_total, size=min(rows_total, DUMP_SAMPLE_ROWS), replace=False))
+    t, v, l = cols
+    arrays = {
+        # frame, then the u128 checksum as four u32 words, least significant first (each exact in float64)
+        "checksums": np.array([[f] + [(c >> s) & 0xFFFFFFFF for s in (0, 32, 64, 96)] for f, c in checksums],
+                              dtype=np.float64).reshape(-1, 5),
+        "sample_rows": rows.astype(np.float64),
+        "alive": eng.read_alive(0, rows_total)[rows].astype(np.float32),
+        "transform": eng.read_component(t, 0, rows_total)[rows].view(np.float32),          # translation | rotation | scale
+        "velocity": eng.read_component(v, 0, rows_total)[rows].view(np.float32),
+        "ttl": eng.read_component(l, 0, rows_total)[rows].view(np.uint64)[:, 0].astype(np.float64),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def generic_world_leg(n):
@@ -857,13 +876,13 @@ def run_cpu_soa_sample(n, d, maxp, rollback_ticks=12):
 
 
 def try_real_reference(n, d, ticks, seed):
-    """BASELINE.md §2(3): where a Rust toolchain and a bevy_ggrs checkout exist (probed at run time — neither does in
-    this image nor on the GPU box), build oracle/ref_harness against the UNMODIFIED reference crate and time the real
-    Bevy SyncTest path.  Returns the harness' timing dict or None."""
+    """BASELINE.md §2(3): where a Rust toolchain and a bevy_ggrs checkout named by BEVY_GGRS_PATH exist (probed at run
+    time), build oracle/ref_harness against the UNMODIFIED reference crate and time the real Bevy SyncTest path.
+    Returns the harness' timing dict or None."""
     import shutil
     import tempfile
-    ref = os.environ.get("BEVY_GGRS_PATH", "/root/reference")
-    if not shutil.which("cargo") or not os.path.exists(os.path.join(ref, "Cargo.toml")):
+    ref = os.environ.get("BEVY_GGRS_PATH", "")
+    if not ref or not shutil.which("cargo") or not os.path.exists(os.path.join(ref, "Cargo.toml")):
         return None
     try:
         tmp = tempfile.mkdtemp()
@@ -918,7 +937,7 @@ def run_reference(args):
         "ms_per_step": r["seconds_per_tick"] * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "u64 (seahash) + f32 + bytes", "data": "synthetic (same generator and seed as the GPU arm)",
         "config": {"workload": args.workload, "entities_per_gpu": n, "check_distance": d, "max_prediction": maxp,
-                   "note": "/root/reference is Rust and cannot be built in this image (no rustc/cargo): this arm times the "
+                   "note": "no Rust toolchain or bevy_ggrs checkout (BEVY_GGRS_PATH) was found: this arm times the "
                            "oracle port, a faithful CPU restatement of the reference's data structures and loops"},
         "cpu_baseline": {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")},
         "e2e": {"value": r["value"], "unit": "rollback frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -928,6 +947,7 @@ def run_reference(args):
 
 
 def main():
+    sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from untouched (it may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=2000)
@@ -940,7 +960,14 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="N > 1: weak = the workload's entity count per GPU; strong = the workload's entity count split over the GPUs (BASELINE C5)")
     ap.add_argument("--trace-out", default="", help="write the device-side launch timeline (CSV) here")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the timed path returned on its last step (checksums + a seeded row sample of the "
+                         "world) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arm only")
     if args.impl == "reference":
         run_reference(args)
     else:

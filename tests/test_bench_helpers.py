@@ -54,6 +54,30 @@ def test_synctest_consistency_check():
     assert not bench.check_synctest_consistency([(1, 5), (1, 7)])
 
 
+def test_dump_outputs_is_exact_seeded_and_float(tmp_path, monkeypatch):
+    """--dump-outputs on a CPU world of the same shape: u128 checksums survive as float64 words bit for bit, the row
+    sample is the same on every run, and every array is float32 or float64."""
+    from oracle_backend import OracleWorld
+    monkeypatch.setattr(bench, "DUMP_SAMPLE_ROWS", 100)
+    orc = OracleWorld(fps=60)
+    cols = bench.build_world(orc, 1000, 4, bench.SEED)
+    checksums = [(3, (1 << 127) | 0x0123456789ABCDEF), (4, 7)]
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), orc, cols, checksums)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["alive.npy", "checksums.npy", "sample_rows.npy", "transform.npy", "ttl.npy", "velocity.npy"]
+    got = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    for n in names:
+        assert np.array_equal(got[n[:-4]], np.load(tmp_path / "b" / n))
+        assert got[n[:-4]].dtype in (np.float32, np.float64)
+    assert [(int(r[0]), sum(int(w) << (32 * i) for i, w in enumerate(r[1:]))) for r in got["checksums"]] == checksums
+    rows = got["sample_rows"].astype(np.int64)
+    assert rows.size == 100 and np.all(np.diff(rows) > 0) and rows[-1] < 1000
+    assert np.array_equal(got["transform"], orc.read_component(cols[0], 0, 1000)[rows].view(np.float32))
+    assert np.array_equal(got["ttl"], orc.read_component(cols[2], 0, 1000)[rows].view(np.uint64)[:, 0].astype(np.float64))
+    orc.close()
+
+
 def test_reference_arm_prints_the_contract_line_on_a_cpu_box():
     """`bench.py --impl reference` = the reference's CPU path (the oracle port here: no cargo, no checkout on the GPU box)
     on host cores, same metric / unit / config keys as our arm, bounded sample, no GPU needed."""
