@@ -85,6 +85,7 @@ PROTOTYPES = {
     "bgr_rollback_component": (C.c_int, [C.c_void_p, C.c_char_p, C.c_uint32, C.c_uint32, u32p]),
     "bgr_checksum_component": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]),
     "bgr_add_system": (C.c_int, [C.c_void_p, C.c_uint32, u32p, C.c_uint32, u32p, C.c_uint32]),
+    "bgr_add_user_system": (C.c_int, [C.c_void_p, C.c_char_p, C.c_char_p, u32p, C.c_uint32, u32p, C.c_uint32]),
     "bgr_build": (C.c_int, [C.c_void_p]),
     "bgr_run_startup_system": (C.c_int, [C.c_void_p, C.c_uint32]),
     "bgr_spawn": (C.c_int, [C.c_void_p, C.c_uint32, u32p]),

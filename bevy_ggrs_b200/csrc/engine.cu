@@ -50,10 +50,21 @@ struct Column {
     uint32_t absent = 0;  // optional column: its absent bit in the per-row mask byte (kernels.cuh row_matches)
 };
 
+// Internal id of a user system (bgr_add_user_system): never a bgr_system value.  It only runs on the registration's own
+// kernel, where its SysSpec::param is its index among the user systems.
+constexpr uint32_t kSysUser = 0x100;
+
 struct SystemReg {
     uint32_t id = 0;
     std::vector<uint32_t> cols, params;
+    std::string name, source;  // user systems: the function's name and its CUDA source
 };
+
+bool has_user_systems(const std::vector<SystemReg>& systems) {
+    for (const SystemReg& sy : systems)
+        if (sy.id == kSysUser) return true;
+    return false;
+}
 
 constexpr uint32_t kReqAdvanceNoBump = 100;  // bgr_advance_world: caller already bumped RollbackFrameCount
 
@@ -259,6 +270,7 @@ namespace {
 // ---------------------------------------------------------------------------------------------
 struct Program {
     Op ops[kMaxOps];
+    int32_t adv_frame[kMaxOps] = {};  // ADVANCE: RollbackFrameCount inside AdvanceWorld
     uint32_t n_ops = 0, n_saves = 0;
     int32_t save_frames[kMaxSaves];
     uint32_t save_totals[kMaxSaves];
@@ -360,6 +372,7 @@ int compile_requests(bgr_engine* e, HostState& s, const bgr_session_info* sess, 
             uint64_t delta = runtime - s.elapsed_ns;
             s.elapsed_ns = runtime;
             op.kind = OP_ADVANCE;
+            pg.adv_frame[pg.n_ops] = s.frame_count;
             op.dt_bits = f32_bits(duration_as_secs_f32(delta));
             op.n_rows = s.n_rows;
             op.call_count = s.call_count;
@@ -758,7 +771,7 @@ void fill_generic_specs(const bgr_engine* e, GenericParams& gp) {
             h.finite = c.hash_flags & BGR_HASH_FLAG_ASSERT_FINITE_F32; h.slot = uint32_t(c.ck_slot);
             h.absent = c.absent;
         }
-    uint32_t counter_index = 0;
+    uint32_t counter_index = 0, user_index = 0;
     for (const SystemReg& sy : e->systems) {
         SysSpec& sp = gp.sys[gp.n_sys++];
         sp.id = sy.id;
@@ -771,25 +784,74 @@ void fill_generic_specs(const bgr_engine* e, GenericParams& gp) {
         case BGR_SYS_DESPAWN_ON_INPUT: sp.param = sy.params[0] | (sy.params[1] << 8); break;
         case BGR_SYS_PARTICLES_UPDATE:
         case BGR_SYS_BOX_MOVE: sp.plane1 = e->cols[sy.cols[1]].first_plane; break;
+        case kSysUser: sp.param = user_index++; break;  // the planes are literals of its dispatcher (jit_specialise)
         default: break;
         }
     }
 }
 
-// NVRTC specialisation of the generic program for this registration (jit.hpp, generic_program_jit.cuh); called by bgr_build
-void jit_specialise(bgr_engine* e) {
+// A C string literal of `text` for a generated static_assert message.
+std::string c_string_literal(const std::string& text) {
+    std::string out = "\"";
+    for (char ch : text) {
+        if (ch == '"' || ch == '\\') out += '\\';
+        out += (ch >= 0x20 && ch < 0x7f) ? ch : '?';
+    }
+    return out + "\"";
+}
+
+// The prelude's part for user systems: the device API, every source in its own namespace with its own line numbers, and
+// one dispatcher per system that binds the function's parameters to the literal word planes of its columns.
+std::string user_systems_prelude(const bgr_engine* e) {
+    std::string pre = "#define BGR_SYS_USER " + std::to_string(kSysUser) + "\n#include \"user_system.cuh\"\n";
+    uint32_t user_index = 0;
+    for (const SystemReg& sy : e->systems) {
+        if (sy.id != kSysUser) continue;
+        const std::string idx = std::to_string(user_index++), ns = "bgr_user_" + idx, fn = ns + "::" + sy.name;
+        pre += "namespace " + ns + " {\n#line 1 \"" + sy.name + "\"\n" + sy.source + "\n}\n";
+        pre += "#line 1 \"bgr_user_dispatch_" + sy.name + "\"\n";
+        pre += "template <> struct bgr_user_system<" + idx + "> {\n";
+        pre += "    using F = bgr_fn_traits<decltype(&" + fn + ")>;\n";
+        pre += "    static_assert(F::arity == " + std::to_string(sy.cols.size()) + ", " +
+               c_string_literal(sy.name + ": takes one component parameter per bound column (" + std::to_string(sy.cols.size()) + ")") + ");\n";
+        std::string planes;
+        for (size_t i = 0; i < sy.cols.size(); ++i) {
+            const Column& c = e->cols[sy.cols[i]];
+            pre += "    static_assert(sizeof(F::elem<" + std::to_string(i) + ">) == " + std::to_string(c.elem_bytes) + ", " +
+                   c_string_literal(sy.name + ": parameter " + std::to_string(i + 1) + " is bound to column '" + c.name + "' of " +
+                                    std::to_string(c.elem_bytes) + " bytes; sizeof of the parameter type differs") + ");\n";
+            planes += (i ? ", " : "") + std::to_string(c.first_plane);
+        }
+        pre += "    template <int N> static __device__ __forceinline__ void run(uint32_t (&w)[N], bool on, const bgr_sys_ctx& base, bool& kill) {\n";
+        pre += "        bgr_sys_ctx ctx = base;\n";
+        for (size_t j = 0; j < 8; ++j)
+            pre += "        ctx.params[" + std::to_string(j) + "] = " + std::to_string(j < sy.params.size() ? sy.params[j] : 0u) + "u;\n";
+        pre += "        bgr_invoke<&" + fn + ">::run<" + planes + ">(w, on, ctx, kill);\n    }\n};\n";
+    }
+    return pre;
+}
+
+// NVRTC specialisation of the generic program for this registration (jit.hpp, generic_program_jit.cuh); called by bgr_build.
+// Registrations of compiled-in systems keep the interpreter when this fails (always BGR_OK).  A registration with user
+// systems has no other kernel: every reason it cannot be compiled is an error of bgr_build.
+int jit_specialise(bgr_engine* e) {
     e->jit = JitKernel{};
     e->jit_small = JitKernel{};
-    if (!e->generic_ok || !e->tune_generic || e->tune_jit == 0 || (e->cfg.flags & BGR_CFG_FORCE_STEPWISE)) return;
-    if (e->bundle_particles && e->tune_bundle) return;  // the bundle has its own kernel
-    if (e->tune_jit == 1 && e->cfg.max_entities < 16384) return;  // small worlds: a tick is launch latency, not worth a compile
+    const bool user = has_user_systems(e->systems);  // bgr_build has refused what user systems cannot run with
+    if (!e->generic_ok || !e->tune_generic || e->tune_jit == 0 || (e->cfg.flags & BGR_CFG_FORCE_STEPWISE)) return BGR_OK;
+    if (e->bundle_particles && e->tune_bundle) return BGR_OK;  // the bundle has its own kernel
+    // small worlds: a tick is launch latency, not worth a compile (user systems run on nothing else)
+    if (!user && e->tune_jit == 1 && e->cfg.max_entities < 16384) return BGR_OK;
     GenericParams gp;
     std::memset(&gp, 0, sizeof gp);
     fill_generic_specs(e, gp);
-    if (e->words < 1 || e->words > 24) return;  // the row has to fit the register file
+    if (e->words < 1 || e->words > 24) return BGR_OK;  // the row has to fit the register file
     for (uint32_t c = 0; c < gp.n_hash; ++c)   // whole-word byte ranges only (every POD of u32 / f32 / u64 fields)
-        if (((gp.hash[c].off | gp.hash[c].len) & 3u) != 0u || gp.hash[c].len < 4 || gp.hash[c].len > 64) return;
+        if (((gp.hash[c].off | gp.hash[c].len) & 3u) != 0u || gp.hash[c].len < 4 || gp.hash[c].len > 64)
+            return user ? fail(BGR_ERR_UNSUPPORTED, "user systems need every checksummed byte range to be 4..64 whole words") : BGR_OK;
+    const std::string user_pre = user ? user_systems_prelude(e) : std::string();
     const int rows = e->tune_jit_rows == 1 || e->tune_jit_rows == 2 ? e->tune_jit_rows : 4;
+    int rc = BGR_OK;
     auto compile = [&](int item_rows, int rows, JitKernel* out) {
         const int threads = item_rows / rows;
         std::string pre;
@@ -815,8 +877,13 @@ void jit_specialise(bgr_engine* e) {
             pre += "{" + u(h.first_plane) + "," + u(h.off) + "," + u(h.len) + "," + u(h.finite) + "," + u(h.slot) + "," + u(h.absent) + "}, ";
         }
         pre += "{0u,0u,0u,0u,0u,0u}\n";
+        pre += user_pre;
         std::string why;
-        if (!jit_generic_program(pre, threads, reinterpret_cast<const void*>(&bgr_abi_version), out, &why) && std::getenv("BGR_JIT_VERBOSE"))
+        bool compile_error = false;
+        const bool ok = jit_generic_program(pre, threads, reinterpret_cast<const void*>(&bgr_abi_version), out, &why, &compile_error);
+        if (!ok && user && rc == BGR_OK)
+            rc = fail(compile_error ? BGR_ERR_INVALID_ARGUMENT : BGR_ERR_UNSUPPORTED, "user systems cannot be compiled: " + why);
+        else if (!ok && std::getenv("BGR_JIT_VERBOSE"))
             std::fprintf(stderr, "[bevy_ggrs_b200] generic program not specialised, the interpreter kernel runs: %s\n", why.c_str());
         out->item_rows = item_rows;
     };
@@ -824,6 +891,8 @@ void jit_specialise(bgr_engine* e) {
     compile(forced ? forced : int(kTileRows), std::min(rows, (forced ? forced : int(kTileRows)) / 32), &e->jit);  // a block is at least one warp
     // worlds of few tiles per SM: quarter-tile items, two rows per thread (measured: profiles/r02_generic_jit_sweep.txt)
     if (!forced && e->jit.fn) compile(128, 2, &e->jit_small);
+    if (rc != BGR_OK) { e->jit = JitKernel{}; e->jit_small = JitKernel{}; }
+    return rc;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -850,6 +919,7 @@ int run_generic(bgr_engine* e, const Program& pg, uint32_t buf) {
     if (pg.has_load || pg.has_advance) gp.flags |= PF_WRITE_LIVE_ACTIVE;
     fill_generic_specs(e, gp);
     std::memcpy(gp.ops, pg.ops, sizeof(Op) * pg.n_ops);
+    std::memcpy(gp.adv_frame, pg.adv_frame, sizeof(int32_t) * pg.n_ops);
     if (e->jit.fn) {  // the registration's own register-resident kernel
         // few tiles per SM: with whole tiles some SMs carry twice the rows of others and set the kernel's duration
         const JitKernel& k = (e->jit_small.fn && gp.n_tiles < 3u * uint32_t(e->num_sms)) ? e->jit_small : e->jit;
@@ -1433,9 +1503,55 @@ BGR_API int bgr_add_system(bgr_engine* e, uint32_t system, const uint32_t* colum
     return BGR_OK;
 }
 
+BGR_API int bgr_add_user_system(bgr_engine* e, const char* name, const char* cuda_source, const uint32_t* columns,
+                                uint32_t n_columns, const uint32_t* params, uint32_t n_params) {
+    if (!e) return fail(BGR_ERR_INVALID_ARGUMENT, "null engine");
+    if (e->built) return fail(BGR_ERR_STATE, "systems must be added before bgr_build");
+    bool ident = name && *name && !(*name >= '0' && *name <= '9');
+    for (const char* q = name; ident && *q; ++q)
+        ident = (*q >= 'a' && *q <= 'z') || (*q >= 'A' && *q <= 'Z') || (*q >= '0' && *q <= '9') || *q == '_';
+    if (!ident) return fail(BGR_ERR_INVALID_ARGUMENT, "user system name must be a C identifier");
+    for (const SystemReg& sy : e->systems)
+        if (sy.id == kSysUser && sy.name == name) return fail(BGR_ERR_INVALID_ARGUMENT, std::string("user system '") + name + "' added twice");
+    if (!cuda_source) return fail(BGR_ERR_INVALID_ARGUMENT, "null user system source");
+    if (std::strlen(cuda_source) > 65536) return fail(BGR_ERR_INVALID_ARGUMENT, "user system source is larger than 64 KB");
+    if (n_columns < 1 || n_columns > 4 || !columns) return fail(BGR_ERR_INVALID_ARGUMENT, "a user system binds 1 to 4 columns");
+    if (n_params > 8 || (n_params && !params)) return fail(BGR_ERR_INVALID_ARGUMENT, "a user system takes at most 8 parameters");
+    SystemReg s;
+    s.id = kSysUser;
+    for (uint32_t i = 0; i < n_columns; ++i) {
+        if (columns[i] >= e->cols.size()) return fail(BGR_ERR_INVALID_ARGUMENT, "system binds an unknown column");
+        for (uint32_t c : s.cols)
+            if (c == columns[i]) return fail(BGR_ERR_INVALID_ARGUMENT, "a user system binds the same column twice");
+        s.cols.push_back(columns[i]);
+    }
+    s.params.assign(params, params + n_params);
+    if (e->systems.size() >= size_t(kMaxGenericSys))
+        return fail(BGR_ERR_CAPACITY, "a registration with user systems holds at most 8 systems in total");
+    s.name = name;
+    s.source = cuda_source;
+    e->systems.push_back(std::move(s));
+    return BGR_OK;
+}
+
 BGR_API int bgr_build(bgr_engine* e) {
     if (!e) return fail(BGR_ERR_INVALID_ARGUMENT, "null engine");
     if (e->built) return fail(BGR_ERR_STATE, "bgr_build called twice");
+    const bool user = has_user_systems(e->systems);
+    if (user) {  // user systems run on the registration's own kernel only (generic_program_jit.cuh)
+        uint32_t words = 0;
+        for (const Column& c : e->cols) words += c.words;
+        if (e->systems.size() > size_t(kMaxGenericSys))
+            return fail(BGR_ERR_CAPACITY, "a registration with user systems holds at most 8 systems in total");
+        if (e->spawn_sys >= 0)
+            return fail(BGR_ERR_UNSUPPORTED, "user systems cannot be combined with spawn_particles (spawning runs on the stepwise and bundle paths)");
+        if (e->cfg.flags & BGR_CFG_FORCE_STEPWISE)
+            return fail(BGR_ERR_UNSUPPORTED, "user systems cannot run with BGR_CFG_FORCE_STEPWISE: they only run on the generated kernel");
+        if (e->tune_jit == 0 || e->tune_generic == 0)
+            return fail(BGR_ERR_UNSUPPORTED, "user systems need the generated kernel (BGR_TUNE_JIT=0 or BGR_TUNE_GENERIC=0 disables it)");
+        if (words > 24)
+            return fail(BGR_ERR_UNSUPPORTED, "user systems need a row of at most 24 words (96 bytes of registered columns)");
+    }
     CUDA_TRY(cudaSetDevice(e->cfg.device));
     uint32_t plane = 0;
     e->n_ck = 0;
@@ -1505,10 +1621,12 @@ BGR_API int bgr_build(bgr_engine* e) {
         for (const SystemReg& sy : e->systems)
             ok = ok && (sy.id == BGR_SYS_U32_ADD || sy.id == BGR_SYS_U32_SATSUB_DESPAWN || sy.id == BGR_SYS_U32_STORE_CALL_COUNT ||
                         sy.id == BGR_SYS_PARTICLES_UPDATE || sy.id == BGR_SYS_PARTICLES_DESPAWN || sy.id == BGR_SYS_BOX_MOVE ||
-                        sy.id == BGR_SYS_DESPAWN_ON_INPUT);
+                        sy.id == BGR_SYS_DESPAWN_ON_INPUT || sy.id == kSysUser);
         e->generic_ok = ok;
     }
-    jit_specialise(e);
+    const int jrc = jit_specialise(e);
+    if (jrc != BGR_OK) return jrc;
+    if (user && !e->jit.fn) return fail(BGR_ERR_UNSUPPORTED, "user systems: the generated kernel was not compiled");
     if (e->jit.fn && e->tune_jit_tiledep) {
         const size_t ni = size_t(e->tiles_for(e->cfg.max_entities)) * 4 + 4;
         CUDA_TRY(cudaMalloc(&e->d_item_done, ni * sizeof(unsigned int)));

@@ -63,6 +63,7 @@ struct GenericParams {
     HashSpec hash[kMaxHashCols];
     SysSpec sys[kMaxGenericSys];
     Op ops[kMaxOps];
+    int32_t adv_frame[kMaxOps];  // ADVANCE: RollbackFrameCount after the frame's increment (user systems' bgr_sys_ctx::frame)
 };
 static_assert(sizeof(GenericParams) <= 4000, "kernel parameter block must fit 4 KB");
 

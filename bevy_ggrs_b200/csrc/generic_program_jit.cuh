@@ -57,7 +57,7 @@ struct JitRows {
 
 // the S-th registered system on the register copy; every system sees the entity's presence as it was before the frame
 template <int S>
-__device__ __forceinline__ void jit_run_systems(JitRows& r, const Op& op, float dt, unsigned long long row0, int B) {
+__device__ __forceinline__ void jit_run_systems(JitRows& r, const Op& op, float dt, int32_t frame, unsigned long long row0, int B) {
     if constexpr (S < kJitNSys) {
         constexpr SysSpec sy = kJitSys[S];
 #pragma unroll
@@ -101,8 +101,20 @@ __device__ __forceinline__ void jit_run_systems(JitRows& r, const Op& op, float 
                     r.w[k][sy.plane1] = __float_as_uint(vx); r.w[k][sy.plane1 + 1] = __float_as_uint(vy); r.w[k][sy.plane1 + 2] = __float_as_uint(vz);
                 }
             }
+#ifdef BGR_SYS_USER  // the prelude registers user systems (user_system.cuh): param = the system's index among them
+            else if constexpr (sy.id == BGR_SYS_USER) {
+                bgr_sys_ctx ctx;
+                ctx.dt = dt;
+                ctx.frame = frame;
+                ctx.n_players = (op.flags >> 8) & 0xFu;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) ctx.inputs[j] = op.inputs[j];
+                ctx.order = row0 + uint32_t(k * B);
+                ::bgr_user_system<int(sy.param)>::run(r.w[k], on, ctx, r.kill[k]);
+            }
+#endif
         }
-        jit_run_systems<S + 1>(r, op, dt, row0, B);
+        jit_run_systems<S + 1>(r, op, dt, frame, row0, B);
     }
 }
 
@@ -202,7 +214,7 @@ extern "C" __global__ void __launch_bounds__(BGR_JIT_ITEM_ROWS / BGR_JIT_ROWS, B
             if (op.kind == OP_ADVANCE) {
 #pragma unroll
                 for (int k = 0; k < kJitRows; ++k) r.kill[k] = false;
-                jit_run_systems<0>(r, op, __uint_as_float(op.dt_bits), row0, B);
+                jit_run_systems<0>(r, op, __uint_as_float(op.dt_bits), p.adv_frame[i], row0, B);
 #pragma unroll
                 for (int k = 0; k < kJitRows; ++k) r.m[k] = r.kill[k] ? 0u : r.m[k];  // despawn commands: after the last system
             } else if (op.kind == OP_SAVE) {

@@ -7,8 +7,10 @@
 // * the kernel sources are the .cuh files next to the shared library (<dir of libbevy_ggrs_b200.so>/csrc, or
 //   $BGR_JIT_SRC_DIR); they are handed to NVRTC as in-memory headers, no include path, no host headers.
 // * compiled programs are cached per process by their generated prelude: engines with the same registration share one.
-// * every failure (no NVRTC, no sources, compile error) is reported once on stderr when BGR_JIT_VERBOSE is set and
-//   otherwise silently falls back to the interpreter; results are identical either way (tests run both).
+// * for registrations of compiled-in systems every failure (no NVRTC, no sources, compile error) is reported once on
+//   stderr when BGR_JIT_VERBOSE is set and otherwise silently falls back to the interpreter; results are identical either
+//   way (tests run both).  A registration with user systems (user_system.cuh) has no interpreter: bgr_build fails with
+//   the reason, and with NVRTC's log for a compile error.
 #pragma once
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -87,33 +89,48 @@ inline std::string source_dir(const void* any_symbol_of_this_library) {
     return (slash == std::string::npos ? std::string(".") : p.substr(0, slash)) + "/csrc";
 }
 
+struct Cached {
+    JitKernel k;               // fn == nullptr: the compile failed
+    std::string why;           // ... and why
+    bool compile_error = false;  // NVRTC rejected the source (as opposed to: no NVRTC, no sources, load failure)
+};
 struct Cache {
     std::mutex mu;
-    std::map<std::string, JitKernel> programs;  // by prelude; a failed compile is cached as fn == nullptr
+    std::map<std::string, Cached> programs;  // by prelude
 };
 inline Cache& cache() { static Cache c; return c; }
 
 }  // namespace jit_detail
 
-// Compile (or fetch) the specialised kernel for `prelude` (the generated #defines).  Returns false and leaves the reason
-// in *why when the interpreter has to be used.
+// Compile (or fetch) the specialised kernel for `prelude` (the generated #defines and user sources).  Returns false and
+// leaves the reason in *why (*compile_error: NVRTC rejected the source, *why holds its log) when it cannot be had.
 inline bool jit_generic_program(const std::string& prelude, int threads, const void* any_symbol_of_this_library, JitKernel* out,
-                                std::string* why) {
+                                std::string* why, bool* compile_error) {
     using namespace jit_detail;
     Cache& c = cache();
     std::lock_guard<std::mutex> lock(c.mu);
+    *compile_error = false;
     auto it = c.programs.find(prelude);
     if (it != c.programs.end()) {
-        *out = it->second;
-        if (!out->fn) *why = "cached failure";
+        *out = it->second.k;
+        *why = it->second.why;
+        *compile_error = it->second.compile_error;
         return out->fn != nullptr;
     }
     JitKernel k;
-    auto finish = [&](bool ok) { c.programs[prelude] = ok ? k : JitKernel{}; if (ok) *out = k; return ok; };
+    auto finish = [&](bool ok) {
+        Cached& e = c.programs[prelude];
+        e.k = ok ? k : JitKernel{};
+        e.why = ok ? std::string() : *why;
+        e.compile_error = *compile_error;
+        if (ok) *out = k;
+        return ok;
+    };
     NvrtcApi& api = nvrtc();
     if (!api.ok) { *why = "libnvrtc not found"; return finish(false); }
     const std::string dir = source_dir(any_symbol_of_this_library);
-    const char* files[] = {"generic_program_jit.cuh", "generic_program.cuh", "kernels.cuh", "seahash.cuh", "tma_copy.cuh", "rtc_prelude.cuh"};
+    const char* files[] = {"generic_program_jit.cuh", "generic_program.cuh", "kernels.cuh", "seahash.cuh", "tma_copy.cuh", "rtc_prelude.cuh",
+                           "user_system.cuh"};
     std::vector<std::string> contents(sizeof files / sizeof *files);
     for (size_t i = 0; i < contents.size(); ++i)
         if (!read_file(dir + "/" + files[i], &contents[i])) { *why = "kernel source not found: " + dir + "/" + files[i]; return finish(false); }
@@ -141,6 +158,7 @@ inline bool jit_generic_program(const std::string& prelude, int threads, const v
         if (n) api.GetProgramLog(prog, &log[0]);
         api.DestroyProgram(&prog);
         *why = "NVRTC compile error:\n" + log;
+        *compile_error = true;
         return finish(false);
     }
     size_t n = 0;

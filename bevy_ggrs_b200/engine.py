@@ -62,6 +62,12 @@ class Engine:
         pa = (C.c_uint32 * max(1, len(params)))(*params)
         self._check(self._lib.bgr_add_system(self._h, system, ca, len(cols), pa, len(params)))
 
+    def add_user_system(self, name: str, source: str, cols: Sequence[int], params: Sequence[int] = ()) -> None:
+        """A GgrsSchedule system of the game's own, as CUDA source (contract: bgr_add_user_system in the header)."""
+        ca = (C.c_uint32 * max(1, len(cols)))(*cols)
+        pa = (C.c_uint32 * max(1, len(params)))(*params)
+        self._check(self._lib.bgr_add_user_system(self._h, name.encode(), source.encode(), ca, len(cols), pa, len(params)))
+
     def build(self) -> None:
         self._check(self._lib.bgr_build(self._h))
 

@@ -69,6 +69,12 @@ struct System {
     std::vector<uint32_t> columns;
     std::vector<uint32_t> params;
 };
+// A GgrsSchedule system of the game's own, as CUDA source (bgr_add_user_system: the contract is in the header).
+struct CudaSystem {
+    std::string name, source;
+    std::vector<uint32_t> columns;
+    std::vector<uint32_t> params;
+};
 
 // A GgrsSchedule system that only touches host-side resources (box_game.rs:146-148 increase_frame_system).
 // Resources are a few bytes and not data-parallel: they stay on the host, this layer rolls them back per frame
@@ -99,7 +105,8 @@ public:
     App& insert_resource(LocalInputs li) { local_inputs_ = std::move(li); return *this; }
     App& add_systems(ReadInputs, std::function<void(App&)> f) { read_inputs_.push_back(std::move(f)); return *this; }
     App& add_systems(Startup, std::function<void(App&)> f) { startup_.push_back(std::move(f)); return *this; }
-    App& add_systems(GgrsSchedule, System s) { systems_.push_back(std::move(s)); return *this; }
+    App& add_systems(GgrsSchedule, System s) { systems_.push_back(std::move(s)); cuda_systems_.emplace_back(); return *this; }
+    App& add_systems(GgrsSchedule, CudaSystem s) { systems_.push_back(System{}); cuda_systems_.push_back(std::move(s)); return *this; }
     App& add_systems(GgrsSchedule, ResourceSystem s) { res_systems_.push_back(std::move(s.fn)); return *this; }
     App& add_observer(std::function<void(const SyncTestMismatch&)> f) { observers_.push_back(std::move(f)); return *this; }
 
@@ -247,8 +254,15 @@ private:
         for (auto& ck : checksums_)
             check(bgr_checksum_component(engine_, ck.first, BGR_HASH_BYTES, ck.second.offset, ck.second.len,
                                          ck.second.assert_finite ? BGR_HASH_FLAG_ASSERT_FINITE_F32 : 0u));
-        for (auto& s : systems_)
-            check(bgr_add_system(engine_, s.id, s.columns.data(), uint32_t(s.columns.size()), s.params.data(), uint32_t(s.params.size())));
+        for (size_t i = 0; i < systems_.size(); ++i) {  // add_systems order, compiled-in and user systems interleaved
+            const System& s = systems_[i];
+            const CudaSystem& u = cuda_systems_[i];
+            if (!u.name.empty())
+                check(bgr_add_user_system(engine_, u.name.c_str(), u.source.c_str(), u.columns.data(), uint32_t(u.columns.size()),
+                                          u.params.data(), uint32_t(u.params.size())));
+            else
+                check(bgr_add_system(engine_, s.id, s.columns.data(), uint32_t(s.columns.size()), s.params.data(), uint32_t(s.params.size())));
+        }
         check(bgr_build(engine_));
         for (auto& f : startup_) f(*this);
     }
@@ -429,6 +443,7 @@ private:
     std::map<std::type_index, uint32_t> columns_;
     std::vector<std::pair<uint32_t, ByteRangeHasher>> checksums_;
     std::vector<System> systems_;
+    std::vector<CudaSystem> cuda_systems_;  // parallel to systems_: a non-empty name marks a user system
     std::vector<std::function<void(App&)>> read_inputs_, startup_;
     std::vector<std::function<void(const SyncTestMismatch&)>> observers_;
     std::optional<Session> session_;

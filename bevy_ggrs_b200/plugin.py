@@ -17,7 +17,8 @@ src/schedule_systems.rs) so that a bevy_ggrs user — and the parity tests — r
 Differences forced by the C ABI (documented in INTEGRATION.md):
   * components are registered by (name, size_of::<T>()) and the per-element hasher is a byte
     range instead of a Rust closure;
-  * GgrsSchedule systems are compiled-in GPU systems named by id;
+  * GgrsSchedule systems are compiled-in GPU systems named by id, or the game's own written as CUDA source
+    (``CudaSystem``);
   * the "World" is the engine: columns live in HBM, the ring of snapshots too.
 
 ``backend`` is any object with the ``bevy_ggrs_b200.engine.Engine`` method surface.  This
@@ -91,6 +92,17 @@ class Session:  # lib.rs:79-86
 class System:
     """A compiled-in GgrsSchedule system: id + the columns it binds + scalar parameters."""
     system: int
+    columns: Sequence[int]
+    params: Sequence[int] = ()
+
+
+@dataclass
+class CudaSystem:
+    """A GgrsSchedule system of the game's own: ``BGR_SYSTEM_FN void name(const bgr_sys_ctx&, bgr_commands&, A&, ...)``
+    in ``source``, one parameter per column of ``columns``, compiled into the registration's kernel at build
+    (``bgr_add_user_system``)."""
+    name: str
+    source: str
     columns: Sequence[int]
     params: Sequence[int] = ()
 
@@ -170,7 +182,10 @@ class App:
             if isinstance(system, ResourceSystem):
                 self._res_systems.append(system.fn)
                 return self
-            assert isinstance(system, System), "GgrsSchedule systems are compiled-in GPU systems or ResourceSystems"
+            if isinstance(system, CudaSystem):
+                self.world.add_user_system(system.name, system.source, list(system.columns), list(system.params))
+                return self
+            assert isinstance(system, System), "GgrsSchedule systems are GPU systems (System, CudaSystem) or ResourceSystems"
             self.world.add_system(system.system, list(system.columns), list(system.params))
         elif schedule is ReadInputs:
             self._read_inputs.append(system)

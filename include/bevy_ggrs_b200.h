@@ -76,7 +76,7 @@ typedef enum bgr_hash_kind { BGR_HASH_NONE = 0, BGR_HASH_BYTES = 1 } bgr_hash_ki
 #define BGR_HASH_FLAG_ASSERT_FINITE_F32 1u /* every 4-byte word in the range must be a finite f32 */
 
 /* Systems that can be added to GgrsSchedule (`add_systems(GgrsSchedule, ...)`, lib.rs:73-74).
- * User closures cannot cross a C ABI; the systems the hot path needs are compiled in. */
+ * These are compiled in; a game's own systems are added as CUDA source with bgr_add_user_system below. */
 typedef enum bgr_system {
     /* update_particles, particles.rs:272-280.  cols = {Transform(40B), Velocity(12B)} */
     BGR_SYS_PARTICLES_UPDATE = 1,
@@ -192,6 +192,40 @@ BGR_API int bgr_checksum_component(bgr_engine* e, uint32_t column, uint32_t hash
 /* add_systems(GgrsSchedule, system) — systems run in insertion order each AdvanceFrame */
 BGR_API int bgr_add_system(bgr_engine* e, uint32_t system, const uint32_t* columns, uint32_t n_columns,
                            const uint32_t* params, uint32_t n_params);
+/* add_systems(GgrsSchedule, NAME) for a system of the game's own, given as CUDA source and compiled into the
+ * registration's own kernel at bgr_build (NVRTC).  It runs in add_systems order, interleaved with the compiled-in systems:
+ *
+ *     struct Velocity { float x, y, z; };
+ *     BGR_SYSTEM_FN void apply_drag(const bgr_sys_ctx& ctx, bgr_commands& cmd, Velocity& v) {
+ *         const float k = bgr_f32(ctx.params[0]);
+ *         v.x = v.x * k; v.y = v.y * k; v.z = v.z * k;
+ *         if (v.x == 0.0f && v.y == 0.0f) cmd.despawn();
+ *     }
+ *
+ *   - signature: `BGR_SYSTEM_FN void NAME(const bgr_sys_ctx&, bgr_commands&, A&, const B&, ...)`, one parameter per bound
+ *     column in binding order (1 to 4).  A..: the game's POD structs, declared in the same source, sizeof == the column's
+ *     elem_bytes (a static_assert naming the column checks it).  `const T&` is `&T` and is never written back; `T&` is
+ *     `&mut T`.  The same column may not be bound twice.
+ *   - entities: every entity that exists and has every bound column (`Query<(&mut A, &B)>`, optional columns included).
+ *     Every system of a frame sees entity presence as it was before the frame.  One entity at a time: no reads of others.
+ *   - cmd.despawn() is deferred to after the last system of the frame, like every despawn command.
+ *   - bgr_sys_ctx: dt (Time<GgrsTime> delta), frame (RollbackFrameCount inside AdvanceWorld, after its `+= 1`),
+ *     n_players / inputs[8] (PlayerInputs<T>), order (the entity's RollbackOrdered index, order_base + row: the player
+ *     handle of box_game-style systems), params[8] (`params`, constant in the generated kernel; bgr_f32 reads one as a
+ *     float).  Input status is not exposed.
+ *   - floating point: + - * / and sqrtf are bit-exact with a CPU build (-fmad=false; g++ -ffp-contract=off on the host);
+ *     transcendentals (powf, sinf, ...) are not.
+ *   - the source has no #include (the API, csrc/user_system.cuh, is already included), no __global__, no __shared__, no
+ *     mutable __device__ globals.  It is compiled inside a namespace of its own (two systems may each declare a
+ *     `struct Velocity`) behind `#line 1 "NAME"`, so compile errors point at the source's own lines.
+ * Checked here: NAME is a C identifier not used by another user system, the source is at most 64 KB, the columns exist
+ * and are distinct, n_params <= 8, at most 8 systems in total, and the call comes before bgr_build.  bgr_build then fails
+ * with BGR_ERR_INVALID_ARGUMENT and NVRTC's log in bgr_last_error() when the source does not compile, and with
+ * BGR_ERR_UNSUPPORTED when the generated kernel cannot be had: no NVRTC or kernel sources, BGR_TUNE_JIT=0 or
+ * BGR_TUNE_GENERIC=0, BGR_CFG_FORCE_STEPWISE, BGR_SYS_PARTICLES_SPAWN in the same registration, or more than 24 words
+ * (96 bytes) of registered columns per entity.  The engine stays destroyable after any of these failures. */
+BGR_API int bgr_add_user_system(bgr_engine* e, const char* name, const char* cuda_source, const uint32_t* columns,
+                                uint32_t n_columns, const uint32_t* params, uint32_t n_params);
 /* end of App::build: allocates live columns + max_depth frame slots in HBM */
 BGR_API int bgr_build(bgr_engine* e);
 /* add_systems(Startup, system): run a registered GgrsSchedule system once, outside the rollback loop
@@ -330,7 +364,7 @@ BGR_API int bgr_slot_bytes(bgr_engine* e, uint64_t* bytes_out);  /* algorithmic 
 BGR_API int bgr_last_path(bgr_engine* e, uint32_t* fused_out);   /* 1 if the last handle_requests used the fused program kernel */
 /* 1 if bgr_build compiled this registration's own kernel (NVRTC specialisation of the generic one-launch program,
  * csrc/generic_program_jit.cuh): every non-bundle request vector then runs on it; 0 = the interpreter kernel (same results).
- * Env BGR_TUNE_JIT: 0 never, 1 (default) engines created for >= 16384 entities, 2 always. */
+ * Env BGR_TUNE_JIT: 0 never, 1 (default) engines created for >= 16384 entities or with user systems, 2 always. */
 BGR_API int bgr_generic_specialised(bgr_engine* e, uint32_t* specialised_out);
 BGR_API int bgr_synchronize(bgr_engine* e);
 BGR_API int bgr_stream(bgr_engine* e, void** stream_out);        /* the cudaStream_t the engine launches on (timing events) */

@@ -46,7 +46,7 @@ use bevy_ggrs_b200_sys as sys;
 use ggrs::{Config, GgrsError, GgrsRequest, SessionState};
 
 pub mod prelude {
-    pub use super::{AddGpuSystems, B200Config, ByteRangeHash, GgrsPlugin, GpuColumn, GpuSystem, RollbackApp, mirror_component};
+    pub use super::{AddGpuSystems, B200Config, ByteRangeHash, CudaSystem, GgrsPlugin, GpuColumn, GpuSystem, RollbackApp, mirror_component};
     pub use bevy_ggrs::{
         AddRollbackCommandExtension, Checksum, ConfirmedFrameCount, GgrsConfig, GgrsSchedule, GgrsTime, LocalInputs, LocalPlayers,
         MaxPredictionWindow, PlayerInputs, ReadInputs, Rollback, RollbackFrameCount, RollbackFrameRate, RollbackId, Session, SyncTestMismatch,
@@ -374,14 +374,37 @@ pub fn handle_requests<C: Config<Input = u8>>(requests: Vec<GgrsRequest<C>>, inf
     world.insert_resource(MaxPredictionWindow(maxp as usize));
 }
 
+/// A GgrsSchedule system of the game's own, written as CUDA source and compiled into the registration's kernel
+/// (`bgr_add_user_system`; the contract is in include/bevy_ggrs_b200.h):
+/// `BGR_SYSTEM_FN void NAME(const bgr_sys_ctx&, bgr_commands&, A&, const B&, ...)`, one parameter per bound column.
+pub struct CudaSystem<'a> {
+    pub name: &'a str,
+    pub source: &'a str,
+    pub columns: &'a [TypeId],
+    pub params: &'a [u32],
+}
+
 /// The GgrsSchedule systems that run on the GPU, in schedule order, each with the component types it binds.
-pub trait AddGpuSystems { fn add_gpu_systems(&mut self, systems: &[(GpuSystem, &[TypeId])]) -> &mut Self; }
+pub trait AddGpuSystems {
+    fn add_gpu_systems(&mut self, systems: &[(GpuSystem, &[TypeId])]) -> &mut Self;
+    fn add_cuda_system(&mut self, system: CudaSystem) -> &mut Self;
+}
 impl AddGpuSystems for App {
     fn add_gpu_systems(&mut self, systems: &[(GpuSystem, &[TypeId])]) -> &mut Self {
         for (s, cols) in systems {
             let ids: Vec<u32> = cols.iter().map(|t| self.world().resource::<Columns>().by_type[t]).collect();
             check(unsafe { sys::bgr_add_system(engine(self.world()), *s as u32, ids.as_ptr(), ids.len() as u32, core::ptr::null(), 0) });
         }
+        self
+    }
+    fn add_cuda_system(&mut self, system: CudaSystem) -> &mut Self {
+        let ids: Vec<u32> = system.columns.iter().map(|t| self.world().resource::<Columns>().by_type[t]).collect();
+        let name = CString::new(system.name).expect("system name without NUL");
+        let source = CString::new(system.source).expect("system source without NUL");
+        check(unsafe {
+            sys::bgr_add_user_system(engine(self.world()), name.as_ptr(), source.as_ptr(), ids.as_ptr(), ids.len() as u32,
+                                     system.params.as_ptr(), system.params.len() as u32)
+        });
         self
     }
 }

@@ -102,6 +102,8 @@ extern "C" {
     pub fn bgr_rollback_component(e: *mut bgr_engine, type_name: *const c_char, elem_bytes: u32, strategy: u32, column_out: *mut u32) -> c_int;
     pub fn bgr_checksum_component(e: *mut bgr_engine, column: u32, hash_kind: u32, byte_offset: u32, byte_len: u32, flags: u32) -> c_int;
     pub fn bgr_add_system(e: *mut bgr_engine, system: u32, columns: *const u32, n_columns: u32, params: *const u32, n_params: u32) -> c_int;
+    pub fn bgr_add_user_system(e: *mut bgr_engine, name: *const c_char, cuda_source: *const c_char, columns: *const u32, n_columns: u32,
+                               params: *const u32, n_params: u32) -> c_int;
     pub fn bgr_build(e: *mut bgr_engine) -> c_int;
     pub fn bgr_run_startup_system(e: *mut bgr_engine, system: u32) -> c_int;
     pub fn bgr_spawn(e: *mut bgr_engine, count: u32, first_row_out: *mut u32) -> c_int;
